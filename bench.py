@@ -23,6 +23,10 @@ cpu_baseline that oracle replay, timed (single thread = the reference's design p
 
 `--impl reference` times the CPU restatement on all host cores (hash-sharded stores, built ONCE at the
 full key count) on the same config instead.
+
+`--dump-outputs DIR` writes the result rows of the last timed tick (at N>1 rank 0's slice; for `--impl reference`
+the last tick of the last step) as DIR/<field>.npy, one float64 array per result field.  The trace is seeded, so
+the same arguments give the same requests and two builds can be compared output for output.
 """
 import argparse
 import glob
@@ -110,6 +114,18 @@ def build_requests(tc, key_hash_of, trace):
     return req
 
 
+def dump_outputs(out_dir, res):
+    """Every field a caller of the timed path receives, one tick of RES_DTYPE rows (2^20 rows: 40 MB).  The fields
+    are integers; float64 holds them exactly below 2^53, which is checked rather than assumed."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("allowed", "status", "remaining", "reset_after_ns", "retry_after_ns"):
+        col = res[name]
+        f = col.astype(np.float64)
+        if not np.array_equal(f.astype(col.dtype), col):
+            raise SystemExit("--dump-outputs: %s has a value float64 cannot hold exactly" % name)
+        np.save(os.path.join(out_dir, name + ".npy"), f)
+
+
 def traffic_from_profiles():
     """DRAM bytes (read + write) of the K1 kernels of ONE tick, summed from the newest committed
     `ncu --set full` raw page under profiles/ (written by tools/ncu_k1_summary.py)."""
@@ -151,11 +167,11 @@ def run_reference(args, rank, world):
     vals = []
     for s in range(W + K):
         tr = traces.config2(n_keys=n_keys, n_ticks=REF_TICKS_PER_STEP, tick_size=TICK, start_tick=s * REF_TICKS_PER_STEP)
-        _, sec = oracle.replay_sharded(stores, tr)               # timed: the decision loops only
+        out, sec = oracle.replay_sharded(stores, tr)             # timed: the decision loops only
         if s >= W:
             vals.append(len(tr) / sec)
-        if time.time() - t0 > 270 and len(vals) >= 3:
-            break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out[-TICK:])
     value = float(np.median(vals))
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
@@ -228,7 +244,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--sustain-sec", type=float, default=0.5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed tick's results as DIR/<field>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -346,6 +366,8 @@ def main():
 
     res_all = d_res.cpu().numpy().view(tc.RES_DTYPE).reshape(W + K, TICK)      # every tick's results, warm-up included
     res_np = res_all[W:]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res_all[W + K - 1])
     n_allowed = int(res_np["allowed"].sum())
     n_ok = int((res_np["status"] == 0).sum())
 

@@ -37,7 +37,8 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        build()
+        if not os.path.exists(_SO):      # loading never recompiles a built library: the tree may be read-only
+            build()
         L = C.CDLL(_SO)
         vp, u64, i64, cp = C.c_void_p, C.c_uint64, C.c_int64, C.c_char_p
         L.ora_create.restype = vp
