@@ -153,7 +153,11 @@ struct P2P {
 struct Scratch {
     Req *drec = nullptr;
     u64 *keys_a = nullptr, *keys_b = nullptr;
-    u32 *hist = nullptr, *tot = nullptr;
+    // one-sweep sort: look-back words [tiles][SORT_MAX_DIGITS]; digit totals, double-buffered by sort
+    // [2][SORT_MAX_PASSES][SORT_MAX_DIGITS], then the tile ticket counter
+    u64 *sort_status = nullptr;
+    u32 *sort_tot = nullptr, *sort_ticket = nullptr;
+    uint32_t sort_seq = 0, sort_tickets = 0, sort_parity = 0;   // last pass sequence number, tickets taken, totals half
     LongRun *long_runs = nullptr, *giant_runs = nullptr;
     u32 *long_count = nullptr;
     cudaEvent_t ev_front = nullptr, ev_mid = nullptr, ev_back = nullptr, ev_fork = nullptr, ev_join = nullptr, ev_join2 = nullptr;
@@ -163,7 +167,7 @@ struct Scratch {
     unsigned char *flags = nullptr;     // [rows] pass-B verdict of rows on shared slots
     u32 *bitmap = nullptr;              // [bm_words] 16-bit occurrence counters of the batch, hashed by slot
     u32 *pend = nullptr;                // [pend_words] 1 bit per entry: the PREVIOUS batch's tail owns a slot of the entry
-    u64 *ctrl_block = nullptr;          // word 0: {tile ticket, residue count}; word 1: {sort barrier, -}; then one status word per tile
+    u64 *ctrl_block = nullptr;          // word 0: {tile ticket, residue count}; then one status word per tile
     uint32_t rows_alloc = 0;
     u32 *h_nres = nullptr;              // pinned: residue size of the set's latest index-order batch (valid after ev_mid)
     bool mid_recorded = false, nres_counted = true;
@@ -538,36 +542,37 @@ static BatchView single_view(const void *d_req, gcra_result *d_res, uint32_t n) 
     return v;
 }
 
-// stable LSD radix sort of `n` (host count) or `*n_dev` (device count) keys on the slot bits; returns the buffer
-// that holds the sorted keys
+static uint32_t sort_tiles_max(const gcra_engine *h) { return (h->max_batch + SORT_TILE - 1) / SORT_TILE; }
+
+// stable LSD radix sort of `n` (host count) or `*n_dev` (device count, at most n_max) keys on the slot bits: one
+// histogram launch for every pass, then one launch per pass; returns the buffer that holds the sorted keys
 static int enqueue_sort(gcra_engine *h, Scratch &sc, uint32_t n_max, const u32 *n_dev, cudaStream_t st, u64 **sorted_out) {
     const uint32_t bits = h->tab.slot_bits;
     const uint32_t passes = (bits + SORT_MAX_BITS - 1) / SORT_MAX_BITS;
-    uint32_t stiles = (n_max + SORT_TILE - 1) / SORT_TILE;
-    if (n_dev) {
-        // fixed grid, all CTAs resident (grid barriers), the kernels loop over the tiles: sized for about twice the
-        // residue the host saw last (a barrier over few CTAs is cheaper), any size is correct
-        const uint32_t guess = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(2ULL * h->last_nres, n_max / 8) + 8 * SORT_TILE, n_max);
-        stiles = std::max<uint32_t>(std::min<uint32_t>((guess + SORT_TILE - 1) / SORT_TILE, 2 * 148), 8);
-    }
+    const uint32_t tiles = (n_max + SORT_TILE - 1) / SORT_TILE;
+    if (passes > SORT_MAX_PASSES) { h->err = "slot bits beyond the sort's passes"; return GCRA_INTERNAL; }
+    u32 *tot = sc.sort_tot + sc.sort_parity * SORT_MAX_PASSES * SORT_MAX_DIGITS;
+    u32 *clear = sc.sort_tot + (sc.sort_parity ^ 1) * SORT_MAX_PASSES * SORT_MAX_DIGITS;
+    sc.sort_parity ^= 1;
+    const uint32_t hgrid = std::min<uint32_t>((n_max + SORT_HIST_KEYS - 1) / SORT_HIST_KEYS, 4 * 148);
+    sort_digits_hist_kernel<<<hgrid, TILE_THREADS, 0, st>>>(sc.keys_a, n_max, n_dev, bits, passes, tot, clear);
     u64 *src = sc.keys_a, *dst = sc.keys_b;
     uint32_t shift = 32;
     for (uint32_t p = 0; p < passes; p++) {
-        uint32_t pb = bits / passes + (p < bits % passes ? 1 : 0);
-        if (n_dev) {
-            // device-side count (the residue): one launch per pass, grid barriers between its phases
-            u32 *bar_cnt = reinterpret_cast<u32 *>(sc.ctrl_block + 1);
-            sort_pass_fused_kernel<<<stiles, TILE_THREADS, 0, st>>>(src, dst, n_dev, shift, pb, sc.hist, sc.tot, bar_cnt, p);
-            h->launches++;
-        } else {
-            sort_hist_kernel<<<stiles, TILE_THREADS, 0, st>>>(src, n_max, n_dev, shift, pb, sc.hist);
-            sort_rowscan_kernel<<<1u << pb, TILE_THREADS, 0, st>>>(sc.hist, n_max, n_dev, sc.tot);
-            sort_scatter_kernel<<<stiles, TILE_THREADS, 0, st>>>(src, dst, n_max, n_dev, shift, pb, sc.hist, sc.tot);
-            h->launches += 3;
+        const uint32_t pb = sort_pass_bits(bits, passes, p);
+        if (sc.sort_seq + 1 >= SORT_SEQ_LIMIT) {
+            // the 31-bit pass sequence number wrapped (once per 2 G passes): forget every look-back word
+            CK(cudaMemsetAsync(sc.sort_status, 0, (size_t)sort_tiles_max(h) * SORT_MAX_DIGITS * sizeof(u64), st));
+            sc.sort_seq = 0;
         }
+        // every CTA takes exactly one ticket, also those beyond a device count
+        sort_onesweep_kernel<<<tiles, TILE_THREADS, 0, st>>>(src, dst, n_max, n_dev, shift, pb, tot + p * SORT_MAX_DIGITS,
+                                                             sc.sort_status, sc.sort_ticket, sc.sort_tickets, ++sc.sort_seq);
+        sc.sort_tickets += tiles;
         std::swap(src, dst);
         shift += pb;
     }
+    h->launches += 1 + passes;
     *sorted_out = src;
     return GCRA_OK;
 }
@@ -615,7 +620,7 @@ static int alloc_index_scratch(gcra_engine *h, Scratch &sc, uint32_t rows) {
     if (tiles > h->max_tiles) h->max_tiles = tiles;
     CK(cudaMalloc(&sc.slot_arr, (size_t)rows * sizeof(u32)));
     CK(cudaMalloc(&sc.flags, (size_t)rows));
-    CK(cudaMalloc(&sc.ctrl_block, ((size_t)h->max_tiles + 2) * sizeof(u64)));
+    CK(cudaMalloc(&sc.ctrl_block, ((size_t)h->max_tiles + 1) * sizeof(u64)));
     if (!sc.h_nres) { CK(cudaMallocHost(&sc.h_nres, sizeof(u32))); *sc.h_nres = 0; }
     if (!sc.bitmap) {
         CK(cudaMalloc(&sc.bitmap, h->bm_words * sizeof(u32)));
@@ -660,7 +665,7 @@ static int enqueue_front(gcra_engine *h, Scratch &sc, const BatchView &v, bool i
         const uint32_t rows = view_max_rows(v);
         const uint32_t tiles = (rows + TILE_THREADS - 1) / TILE_THREADS;
         const uint32_t grid = std::min<uint32_t>(tiles, h->grid_probe[compact ? 1 : 0]);    // persistent, software-pipelined CTAs
-        CK(cudaMemsetAsync(sc.ctrl_block, 0, ((size_t)h->max_tiles + 2) * sizeof(u64), st));
+        CK(cudaMemsetAsync(sc.ctrl_block, 0, ((size_t)h->max_tiles + 1) * sizeof(u64), st));
         if (timed) CK(cudaEventRecord(h->evd[0], st));
         if (compact)
             probe_kernel<true><<<grid, TILE_THREADS, 0, st>>>(h->tab, v, h->d_pol, h->npol, now_batch, sc.slot_arr, sc.bitmap,
@@ -704,7 +709,7 @@ static int enqueue_mid_index(gcra_engine *h, Scratch &sc, Scratch &next, const B
     const uint32_t grid = std::min<uint32_t>((rows + TILE_THREADS - 1) / TILE_THREADS, h->grid_decide[compact ? 1 : 0]);   // persistent CTAs
     const uint32_t rgrid = std::min<uint32_t>((rows + RES_TILE - 1) / RES_TILE + v.nseg, 6 * 148);
     u32 *ctrl = reinterpret_cast<u32 *>(sc.ctrl_block);
-    u64 *status = sc.ctrl_block + 2;
+    u64 *status = sc.ctrl_block + 1;
     if (compact) {
         decide_index_kernel<true><<<grid, TILE_THREADS, 0, st>>>(h->tab, v, h->d_pol, h->npol, now_batch, sc.slot_arr,
                                                                  sc.bitmap, sc.pend, h->bm_mask, sc.flags, h->epoch, hp, h->dbg);
@@ -928,7 +933,7 @@ static void preload(K kernel) {
 static void preload_kernels() {
     preload(ingest_kernel<false>); preload(ingest_kernel<true>);
     preload(small_batch_kernel<false>); preload(small_batch_kernel<true>);
-    preload(sort_hist_kernel); preload(sort_rowscan_kernel); preload(sort_scatter_kernel); preload(sort_pass_fused_kernel);
+    preload(sort_digits_hist_kernel); preload(sort_onesweep_kernel);
     preload(decide_kernel<false>); preload(decide_kernel<true>);
     preload(decide_runs_kernel<1, false>); preload(decide_runs_kernel<CLUSTER_CTAS, false>);
     preload(decide_runs_kernel<1, true>); preload(decide_runs_kernel<CLUSTER_CTAS, true>);
@@ -1000,7 +1005,7 @@ int32_t gcra_create(const gcra_config *cfg, gcra_engine **out) {
         return GCRA_INTERNAL;
     }
     const size_t mb = h->max_batch;
-    const uint32_t stiles = (uint32_t)((mb + SORT_TILE - 1) / SORT_TILE);
+    const uint32_t stiles = sort_tiles_max(h);
     {
         // index-order pipeline: hashed batch counters (16 bits) and pend bits, 8 entries per row of the largest
         // batch (n distinct slots share their entry with probability ~1/8), 64 K .. 16 M entries
@@ -1038,8 +1043,10 @@ int32_t gcra_create(const gcra_config *cfg, gcra_engine **out) {
         ok = cudaMalloc(&sc.drec, mb * sizeof(Req)) == cudaSuccess &&
              cudaMalloc(&sc.keys_a, mb * sizeof(u64)) == cudaSuccess &&
              cudaMalloc(&sc.keys_b, mb * sizeof(u64)) == cudaSuccess &&
-             cudaMalloc(&sc.hist, (size_t)SORT_MAX_DIGITS * stiles * sizeof(u32)) == cudaSuccess &&
-             cudaMalloc(&sc.tot, SORT_MAX_DIGITS * sizeof(u32)) == cudaSuccess &&
+             cudaMalloc(&sc.sort_status, (size_t)SORT_MAX_DIGITS * stiles * sizeof(u64)) == cudaSuccess &&
+             cudaMemset(sc.sort_status, 0, (size_t)SORT_MAX_DIGITS * stiles * sizeof(u64)) == cudaSuccess &&
+             cudaMalloc(&sc.sort_tot, (2 * SORT_MAX_PASSES * SORT_MAX_DIGITS + 1) * sizeof(u32)) == cudaSuccess &&
+             cudaMemset(sc.sort_tot, 0, (2 * SORT_MAX_PASSES * SORT_MAX_DIGITS + 1) * sizeof(u32)) == cudaSuccess &&
              cudaMalloc(&sc.long_runs, (mb / LONG_RUN_MIN + 1) * sizeof(LongRun)) == cudaSuccess &&
              cudaMalloc(&sc.giant_runs, (mb / GIANT_RUN_MIN + 1) * sizeof(LongRun)) == cudaSuccess &&
              cudaMalloc(&sc.long_count, 2 * sizeof(u32)) == cudaSuccess &&
@@ -1049,6 +1056,7 @@ int32_t gcra_create(const gcra_config *cfg, gcra_engine **out) {
              cudaEventCreateWithFlags(&sc.ev_fork, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&sc.ev_join, cudaEventDisableTiming) == cudaSuccess &&
              cudaEventCreateWithFlags(&sc.ev_join2, cudaEventDisableTiming) == cudaSuccess;
+        if (ok) sc.sort_ticket = sc.sort_tot + 2 * SORT_MAX_PASSES * SORT_MAX_DIGITS;
         ok = ok && alloc_index_scratch(h, sc, h->max_batch) == GCRA_OK;
     }
     if (!ok) return fail("scratch allocation", cudaGetLastError());
@@ -1113,7 +1121,7 @@ void gcra_destroy(gcra_engine *h) {
     }
     cudaFree(h->tab.keys); cudaFree(h->tab.state); cudaFree(h->tab.ei); cudaFree(h->tab.mark); cudaFree(h->tab.counters);
     for (auto &sc : h->scr) {
-        cudaFree(sc.drec); cudaFree(sc.keys_a); cudaFree(sc.keys_b); cudaFree(sc.hist); cudaFree(sc.tot);
+        cudaFree(sc.drec); cudaFree(sc.keys_a); cudaFree(sc.keys_b); cudaFree(sc.sort_status); cudaFree(sc.sort_tot);
         cudaFree(sc.long_runs); cudaFree(sc.giant_runs); cudaFree(sc.long_count);
         cudaFree(sc.slot_arr); cudaFree(sc.flags); cudaFree(sc.bitmap); cudaFree(sc.pend); cudaFree(sc.ctrl_block);
         cudaFreeHost(sc.h_nres);

@@ -2,7 +2,7 @@
 //
 //   K1a ingest  : bulk-async (TMA, UBLKCP) staging of a request tile into shared memory, per-request
 //                 validation + parameter derivation (rate_limiter.rs:111-122), key -> slot probe/claim
-//   K1b order   : stable LSD radix sort of (slot, index) so that requests on one key are adjacent and
+//   K1b order   : stable one-sweep LSD radix sort of (slot, index) so that requests on one key are adjacent and
 //                 in index order -- the reference applies requests strictly one at a time
 //                 (throttlecrab-server/src/actor.rs:217-236)
 //   K1c decide  : warp-cooperative GCRA compare-and-update (rate_limiter.rs:150-248); duplicates of a
@@ -174,15 +174,32 @@ ingest_kernel(Table t, const void *__restrict__ req_base, const PolicyDerived *_
 }
 
 // ---------------------------------------------------------------------------------------------
-// K1b: stable LSD radix sort on the slot bits of (slot << 32 | index)
+// K1b: stable LSD radix sort on the slot bits of (slot << 32 | index), one sweep per pass
 // ---------------------------------------------------------------------------------------------
+// One launch reads the keys once and builds the digit histograms of every pass (sort_digits_hist_kernel).  Then
+// one launch per pass (sort_onesweep_kernel): a CTA ranks one tile of keys in shared memory, publishes the tile's
+// count of every digit, finds the counts of all tiles before it by decoupled look-back, and scatters.  A CTA takes
+// its tile from a ticket counter, so tiles are handed out in the order CTAs start: a tile only ever waits on tiles
+// that running (or finished) CTAs hold, and those publish their counts before they wait on anything.  No grid
+// barrier, no assumption about how many CTAs are resident.
 #ifndef GCRA_SORT_ITEMS
-#define GCRA_SORT_ITEMS 4
+#define GCRA_SORT_ITEMS 16
 #endif
 constexpr int SORT_ITEMS = GCRA_SORT_ITEMS;                // items per thread
-constexpr int SORT_TILE = TILE_THREADS * SORT_ITEMS;       // 1024 keys per CTA
+constexpr int SORT_TILE = TILE_THREADS * SORT_ITEMS;       // 4096 keys per tile
+// CTAs per SM of the one-sweep kernel: 2 x 148 SMs hold all 256 tiles of a 2^20-key sort at once, with registers
+// for every thread's 16 keys (no spills)
+constexpr int SORT_MIN_CTAS = 2;
 constexpr int SORT_MAX_BITS = 9;
 constexpr int SORT_MAX_DIGITS = 1 << SORT_MAX_BITS;
+constexpr int SORT_MAX_PASSES = 4;                         // slot_bits <= 32: at most 4 passes of 8 bits
+constexpr int SORT_HIST_KEYS = 2 * SORT_TILE;              // keys per CTA of the histogram kernel
+constexpr int SORT_LOOKBACK = 4;                           // predecessor words read per look-back step
+
+// digit width of pass p: `bits` slot bits over `passes` passes, the first bits % passes passes one bit wider
+__host__ __device__ __forceinline__ u32 sort_pass_bits(u32 bits, u32 passes, u32 p) {
+    return bits / passes + (p < bits % passes ? 1u : 0u);
+}
 
 // block-wide exclusive scan of one value per thread (warp shuffles + one shared-memory hop);
 // returns the exclusive prefix, the block total in *total
@@ -211,156 +228,181 @@ __device__ __forceinline__ u32 block_exclusive_scan(u32 v, u32 *part, u32 *total
     return before + inc - v;
 }
 
-// All three kernels loop over the tiles (grid-stride), and take the element count either from the host
-// (`n`) or -- when `n_dev` is given -- from device memory: the residue of the index-order pipeline is only
-// known on the device, its kernels are launched with a fixed grid.
+// The sort kernels take the element count either from the host (`n`) or -- when `n_dev` is given -- from device
+// memory: the residue of the index-order pipeline is only known on the device, its launches are sized for the
+// largest residue and the tiles beyond the count exit.
 __device__ __forceinline__ u32 sort_count(u32 n, const u32 *__restrict__ n_dev) { return n_dev ? *n_dev : n; }
 
-// the three phases of one pass; hist / tot are read through L2 (__ldcg): the fused kernel below reads what
-// OTHER CTAs of the same launch wrote a phase earlier
-__device__ __forceinline__ void sort_hist_body(u32 *h, const u64 *__restrict__ in, u32 n, u32 shift, u32 bits,
-                                               u32 *__restrict__ hist) {
-    const u32 num_tiles = (n + SORT_TILE - 1) / SORT_TILE;
-    const u32 nd = 1u << bits, mask = nd - 1;
-    for (u32 tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        for (u32 d = threadIdx.x; d < nd; d += TILE_THREADS) h[d] = 0;
-        __syncthreads();
-        const u32 base = tile * SORT_TILE;
+// tot: this sort's digit totals [SORT_MAX_PASSES][SORT_MAX_DIGITS], zero on entry.  clear: the other half of the
+// double buffer, the totals of the previous sort on this scratch set (every pass of it has finished): zeroed here
+// for the next sort, so no memset is needed.
+__global__ void __launch_bounds__(TILE_THREADS)
+sort_digits_hist_kernel(const u64 *__restrict__ in, u32 n_host, const u32 *__restrict__ n_dev, u32 bits, u32 passes,
+                        u32 *__restrict__ tot, u32 *__restrict__ clear) {
+    __shared__ u32 h[SORT_MAX_PASSES * SORT_MAX_DIGITS];
+    for (u32 i = threadIdx.x; i < SORT_MAX_PASSES * SORT_MAX_DIGITS; i += TILE_THREADS) {
+        h[i] = 0;
+        if (blockIdx.x == 0) clear[i] = 0;
+    }
+    u32 shift[SORT_MAX_PASSES], mask[SORT_MAX_PASSES];
+    {
+        u32 s = 32;
+#pragma unroll
+        for (int p = 0; p < SORT_MAX_PASSES; p++) {
+            const u32 pb = (u32)p < passes ? sort_pass_bits(bits, passes, p) : 0;
+            shift[p] = s;
+            mask[p] = (1u << pb) - 1;
+            s += pb;
+        }
+    }
+    __syncthreads();
+    const u32 n = sort_count(n_host, n_dev);
+    for (u32 base = blockIdx.x * SORT_TILE; base < n; base += gridDim.x * SORT_TILE) {
+        u64 key[SORT_ITEMS];
 #pragma unroll
         for (int k = 0; k < SORT_ITEMS; k++) {
-            u32 i = base + k * TILE_THREADS + threadIdx.x;
-            if (i < n) atomicAdd(&h[(u32)(in[i] >> shift) & mask], 1u);
+            const u32 i = base + k * TILE_THREADS + threadIdx.x;
+            key[k] = i < n ? in[i] : 0;
         }
-        __syncthreads();
-        for (u32 d = threadIdx.x; d < nd; d += TILE_THREADS) hist[(size_t)d * num_tiles + tile] = h[d];
-        __syncthreads();
+#pragma unroll
+        for (int k = 0; k < SORT_ITEMS; k++) {
+            if (base + k * TILE_THREADS + threadIdx.x >= n) continue;
+#pragma unroll
+            for (int p = 0; p < SORT_MAX_PASSES; p++)
+                if ((u32)p < passes) atomicAdd(&h[p * SORT_MAX_DIGITS + ((u32)(key[k] >> shift[p]) & mask[p])], 1u);
+        }
     }
+    __syncthreads();
+    for (u32 i = threadIdx.x; i < passes * SORT_MAX_DIGITS; i += TILE_THREADS)
+        if (h[i]) atomicAdd(&tot[i], h[i]);
 }
 
-// exclusive scan of digit `digit`'s per-tile counts, digit total to tot[digit] (the whole CTA works on it)
-__device__ __forceinline__ void sort_rowscan_body(u32 *part, u32 *__restrict__ hist, u32 n, u32 digit, u32 *__restrict__ tot) {
-    const u32 num_tiles = (n + SORT_TILE - 1) / SORT_TILE;
-    u32 *row = hist + (size_t)digit * num_tiles;
-    const u32 per = (num_tiles + TILE_THREADS - 1) / TILE_THREADS;
-    const u32 lo = min(threadIdx.x * per, num_tiles), hi = min(lo + per, num_tiles);
-    u32 s = 0;
-    for (u32 i = lo; i < hi; i++) s += __ldcg(&row[i]);
-    u32 total;
-    u32 acc = block_exclusive_scan(s, part, &total);
-    for (u32 i = lo; i < hi; i++) { u32 v = __ldcg(&row[i]); row[i] = acc; acc += v; }
-    if (threadIdx.x == 0) tot[digit] = total;
-    __syncthreads();   // `part` is reused by the next call
+// Look-back status of (tile, digit) in one 64-bit word: [63:33] the pass's sequence number, [32] 1 = inclusive
+// prefix over tiles 0..tile, 0 = this tile's count only, [31:0] the count.  Every pass of every sort on a scratch
+// set gets a new sequence number (never 0), so words left by earlier passes read as "not published yet" and the
+// array is never cleared between passes.
+constexpr u64 SORT_STATUS_INCL = 1ULL << 32;
+constexpr u32 SORT_SEQ_LIMIT = 1u << 31;
+__device__ __forceinline__ u64 sort_status(u32 seq, bool incl, u32 count) {
+    return ((u64)seq << 33) | (incl ? SORT_STATUS_INCL : 0) | count;
+}
+__device__ __forceinline__ u64 ld_relaxed_gpu(const u64 *p) {
+    u64 v;
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_relaxed_gpu(u64 *p, u64 v) {
+    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
 
-struct SortScatterSmem {
-    u32 cnt[TILE_THREADS / 32][SORT_MAX_DIGITS];   // per-warp digit counters -> per-warp offsets
-    u32 gbase[SORT_MAX_DIGITS];                    // global base of (digit, this tile)
+struct SortOnesweepSmem {
+    u32 cnt[TILE_THREADS / 32][SORT_MAX_DIGITS];   // per-warp digit counters -> per-warp offsets inside the tile
+    u32 gbase[SORT_MAX_DIGITS];                    // output position of (digit, this tile)
     u32 part[TILE_THREADS / 32];
+    u32 tile;
 };
 
-__device__ __forceinline__ void sort_scatter_body(SortScatterSmem &sm, const u64 *__restrict__ in, u64 *__restrict__ outk,
-                                                  u32 n, u32 shift, u32 bits, const u32 *__restrict__ hist,
-                                                  const u32 *__restrict__ tot) {
+// One pass.  tot: the digit totals of this pass (sort_digits_hist_kernel); status: [tiles][SORT_MAX_DIGITS] look-back
+// words; the CTA's tile is atomicAdd(ticket) - ticket_base (the host knows how many tickets earlier launches took).
+__global__ void __launch_bounds__(TILE_THREADS, SORT_MIN_CTAS)
+sort_onesweep_kernel(const u64 *__restrict__ in, u64 *__restrict__ outk, u32 n_host, const u32 *__restrict__ n_dev,
+                     u32 shift, u32 bits, const u32 *__restrict__ tot, u64 *__restrict__ status, u32 *__restrict__ ticket,
+                     u32 ticket_base, u32 seq) {
     constexpr int NW = TILE_THREADS / 32;
-    const u32 num_tiles = (n + SORT_TILE - 1) / SORT_TILE;
-    if (blockIdx.x >= num_tiles) return;       // uniform over the CTA
+    __shared__ SortOnesweepSmem sm;
+    if (threadIdx.x == 0) sm.tile = atomicAdd(ticket, 1u) - ticket_base;
     const u32 nd = 1u << bits, mask = nd - 1;
+    for (u32 d = threadIdx.x; d < nd; d += TILE_THREADS) {
+#pragma unroll
+        for (int x = 0; x < NW; x++) sm.cnt[x][d] = 0;
+    }
+    __syncthreads();
+    const u32 n = sort_count(n_host, n_dev);
+    const u32 tile = sm.tile;
+    if ((u64)tile * SORT_TILE >= n) return;       // uniform over the CTA
     const u32 w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // exclusive scan of the digit totals (nd <= 512: two consecutive digits per thread), once per CTA
+    const u32 lt = (1u << lane) - 1;
+    // warp w owns the tile elements [w * 32 * SORT_ITEMS, (w + 1) * 32 * SORT_ITEMS): item k, lane l -> k * 32 + l,
+    // in index order, and ranks them in that order: the sort is stable
+    const u32 base = tile * SORT_TILE + w * (32 * SORT_ITEMS);
+    u64 key[SORT_ITEMS];
+    u32 dig[SORT_ITEMS], rank[SORT_ITEMS];
+#pragma unroll
+    for (int k = 0; k < SORT_ITEMS; k++) {
+        const u32 i = base + k * 32 + lane;
+        key[k] = i < n ? in[i] : 0;
+    }
+#pragma unroll
+    for (int k = 0; k < SORT_ITEMS; k++) {
+        const bool valid = base + k * 32 + lane < n;
+        dig[k] = (u32)(key[k] >> shift) & mask;
+        const u32 peers = __match_any_sync(0xffffffffu, valid ? dig[k] : (0x80000000u | lane));
+        const u32 before = valid ? sm.cnt[w][dig[k]] : 0;
+        rank[k] = before + __popc(peers & lt);
+        __syncwarp();
+        if (valid && (peers & lt) == 0) sm.cnt[w][dig[k]] = before + __popc(peers);
+        __syncwarp();
+    }
+    // global start of every digit: exclusive scan of the digit totals, two consecutive digits per thread
+    // (nd <= 512); the scan's barriers also complete the per-warp counters
     const u32 d0 = 2 * threadIdx.x, d1 = d0 + 1;
-    const u32 t0 = d0 < nd ? __ldcg(&tot[d0]) : 0, t1 = d1 < nd ? __ldcg(&tot[d1]) : 0;
+    const u32 t0 = d0 < nd ? tot[d0] : 0, t1 = d1 < nd ? tot[d1] : 0;
     u32 total;
     const u32 ex = block_exclusive_scan(t0 + t1, sm.part, &total);
-    const u32 lt = (1u << lane) - 1;
-    for (u32 tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        for (u32 d = threadIdx.x; d < nd; d += TILE_THREADS) {
+    // per digit: exclusive scan over the warps -> the tile's count, published at once
+    u32 agg0 = 0, agg1 = 0;
+    if (d0 < nd) {
 #pragma unroll
-            for (int x = 0; x < NW; x++) sm.cnt[x][d] = 0;
-        }
-        if (d0 < nd) sm.gbase[d0] = ex + __ldcg(&hist[(size_t)d0 * num_tiles + tile]);
-        if (d1 < nd) sm.gbase[d1] = ex + t0 + __ldcg(&hist[(size_t)d1 * num_tiles + tile]);
-        __syncthreads();
-        // warp w owns tile elements [w*128, w*128+128): item k, lane l -> w*128 + k*32 + l (index order)
-        const u32 base = tile * SORT_TILE + w * (32 * SORT_ITEMS);
-        u64 key[SORT_ITEMS];
-        u32 dig[SORT_ITEMS], rank[SORT_ITEMS];
-#pragma unroll
-        for (int k = 0; k < SORT_ITEMS; k++) {
-            u32 i = base + k * 32 + lane;
-            bool valid = i < n;
-            key[k] = valid ? in[i] : 0;
-            dig[k] = (u32)(key[k] >> shift) & mask;
-            u32 peers = __match_any_sync(0xffffffffu, valid ? dig[k] : (0x80000000u | lane));
-            u32 before = valid ? sm.cnt[w][dig[k]] : 0;
-            rank[k] = before + __popc(peers & lt);
-            __syncwarp();
-            if (valid && (peers & lt) == 0) sm.cnt[w][dig[k]] = before + __popc(peers);
-            __syncwarp();
-        }
-        __syncthreads();
-        // per digit: exclusive scan over the warps
-        for (u32 d = threadIdx.x; d < nd; d += TILE_THREADS) {
-            u32 acc = 0;
-#pragma unroll
-            for (int x = 0; x < NW; x++) { u32 v = sm.cnt[x][d]; sm.cnt[x][d] = acc; acc += v; }
-        }
-        __syncthreads();
-#pragma unroll
-        for (int k = 0; k < SORT_ITEMS; k++) {
-            u32 i = base + k * 32 + lane;
-            if (i < n) outk[sm.gbase[dig[k]] + sm.cnt[w][dig[k]] + rank[k]] = key[k];
-        }
-        __syncthreads();
+        for (int x = 0; x < NW; x++) { const u32 v = sm.cnt[x][d0]; sm.cnt[x][d0] = agg0; agg0 += v; }
     }
-}
-
-__global__ void __launch_bounds__(TILE_THREADS)
-sort_hist_kernel(const u64 *__restrict__ in, u32 n_host, const u32 *__restrict__ n_dev, u32 shift, u32 bits,
-                 u32 *__restrict__ hist) {
-    __shared__ u32 h[SORT_MAX_DIGITS];
-    sort_hist_body(h, in, sort_count(n_host, n_dev), shift, bits, hist);
-}
-
-// one CTA per digit
-__global__ void __launch_bounds__(TILE_THREADS)
-sort_rowscan_kernel(u32 *__restrict__ hist, u32 n_host, const u32 *__restrict__ n_dev, u32 *__restrict__ tot) {
-    __shared__ u32 part[TILE_THREADS / 32];
-    sort_rowscan_body(part, hist, sort_count(n_host, n_dev), blockIdx.x, tot);
-}
-
-__global__ void __launch_bounds__(TILE_THREADS)
-sort_scatter_kernel(const u64 *__restrict__ in, u64 *__restrict__ outk, u32 n_host, const u32 *__restrict__ n_dev,
-                    u32 shift, u32 bits, const u32 *__restrict__ hist, const u32 *__restrict__ tot) {
-    __shared__ SortScatterSmem sm;
-    sort_scatter_body(sm, in, outk, sort_count(n_host, n_dev), shift, bits, hist, tot);
-}
-
-// One radix pass in ONE launch for small inputs (the residue of the index-order pipeline: its nine launches of a
-// few microseconds each were pure launch latency).  All CTAs are resident (the host launches at most what fits),
-// the phases are separated by a grid-wide barrier on a counter that the host zeroes once per batch: the barrier
-// after phase p of pass q is complete when the counter reaches (2 q + p + 1) * gridDim.x.
-__device__ __forceinline__ void grid_barrier(u32 *cnt, u32 target) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        atomicAdd(cnt, 1u);
-        while (*reinterpret_cast<volatile u32 *>(cnt) < target) { }
-        __threadfence();
+    if (d1 < nd) {
+#pragma unroll
+        for (int x = 0; x < NW; x++) { const u32 v = sm.cnt[x][d1]; sm.cnt[x][d1] = agg1; agg1 += v; }
     }
+    u64 *row = status + (size_t)tile * SORT_MAX_DIGITS;
+    if (d0 < nd) st_relaxed_gpu(&row[d0], sort_status(seq, tile == 0, agg0));
+    if (d1 < nd) st_relaxed_gpu(&row[d1], sort_status(seq, tile == 0, agg1));
+    // look-back: add the predecessors' counts until one has published its inclusive prefix.  SORT_LOOKBACK words
+    // of both digits are read at once: a tile that starts with hundreds of others before it reaches an inclusive
+    // prefix in a few L2 round trips instead of one per predecessor.
+    u32 pre0 = 0, pre1 = 0;
+    if (tile > 0) {
+        bool done0 = d0 >= nd, done1 = d1 >= nd;
+        u32 next0 = tile, next1 = tile;            // tiles [next, tile) are summed
+        while (!(done0 && done1)) {
+            u64 s0[SORT_LOOKBACK], s1[SORT_LOOKBACK];
+#pragma unroll
+            for (int j = 0; j < SORT_LOOKBACK; j++) {
+                s0[j] = !done0 && (u32)j < next0 ? ld_relaxed_gpu(status + (size_t)(next0 - 1 - j) * SORT_MAX_DIGITS + d0) : 0;
+                s1[j] = !done1 && (u32)j < next1 ? ld_relaxed_gpu(status + (size_t)(next1 - 1 - j) * SORT_MAX_DIGITS + d1) : 0;
+            }
+            bool go0 = !done0, go1 = !done1;       // stop at the first word not published yet, retry from there
+#pragma unroll
+            for (int j = 0; j < SORT_LOOKBACK; j++) {
+                go0 = go0 && (u32)(s0[j] >> 33) == seq;
+                if (go0) {
+                    pre0 += (u32)s0[j];
+                    next0--;
+                    if (s0[j] & SORT_STATUS_INCL) { done0 = true; go0 = false; }
+                }
+                go1 = go1 && (u32)(s1[j] >> 33) == seq;
+                if (go1) {
+                    pre1 += (u32)s1[j];
+                    next1--;
+                    if (s1[j] & SORT_STATUS_INCL) { done1 = true; go1 = false; }
+                }
+            }
+        }
+        if (d0 < nd) st_relaxed_gpu(&row[d0], sort_status(seq, true, pre0 + agg0));
+        if (d1 < nd) st_relaxed_gpu(&row[d1], sort_status(seq, true, pre1 + agg1));
+    }
+    if (d0 < nd) sm.gbase[d0] = ex + pre0;
+    if (d1 < nd) sm.gbase[d1] = ex + t0 + pre1;
     __syncthreads();
-}
-
-__global__ void __launch_bounds__(TILE_THREADS)
-sort_pass_fused_kernel(const u64 *__restrict__ in, u64 *__restrict__ outk, const u32 *__restrict__ n_dev, u32 shift,
-                       u32 bits, u32 *__restrict__ hist, u32 *__restrict__ tot, u32 *__restrict__ bar_cnt, u32 pass) {
-    __shared__ SortScatterSmem sm;
-    const u32 n = *n_dev;
-    if (n == 0) return;                                   // uniform over the grid: nobody enters a barrier
-    sort_hist_body(sm.gbase, in, n, shift, bits, hist);   // (gbase doubles as the histogram of phase 1)
-    grid_barrier(bar_cnt, (2 * pass + 1) * gridDim.x);
-    for (u32 d = blockIdx.x; d < (1u << bits); d += gridDim.x) sort_rowscan_body(sm.part, hist, n, d, tot);
-    grid_barrier(bar_cnt, (2 * pass + 2) * gridDim.x);
-    sort_scatter_body(sm, in, outk, n, shift, bits, hist, tot);
+#pragma unroll
+    for (int k = 0; k < SORT_ITEMS; k++) {
+        if (base + k * 32 + lane < n) outk[sm.gbase[dig[k]] + sm.cnt[w][dig[k]] + rank[k]] = key[k];
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
